@@ -407,6 +407,44 @@ def _params_checksum(tr):
     return int(((a * w).sum() + 31 * (b * w).sum()).item())
 
 
+DUMP_BYTES = 64 << 20
+
+
+def _dump_outputs(tr, out_dir):
+    """Writes what the last timed update left for its caller as out_dir/<name>.npy (float32, or float64 for the episode log):
+    parameters, Adam moments, loss terms, gradient norm, the rollout planes, advantages / returns and the finished-episode log.
+    When the [T+1][N] planes of all envs would pass half of DUMP_BYTES, they are kept for a fixed, seeded sample of env
+    columns (`env_index`) and the episode log for those envs only.  Reads the episode log, which clears it."""
+    import numpy as np
+    import torch
+    torch.cuda.synchronize()
+    T1, N = tr.rewards.shape
+    O = tr.env.obs_dim
+    per_env = T1 * (O + 7) * 4                      # observations + 7 one-value planes, float32
+    cols = np.arange(N)
+    if N * per_env > DUMP_BYTES // 2:
+        cols = np.sort(np.random.default_rng(0).choice(N, (DUMP_BYTES // 2) // per_env, replace=False))
+    sel = torch.from_numpy(cols).to(tr.device)
+    planes = {"observations": tr.observations[:, :, :O], "actions": tr.actions, "log_probs": tr.log_probs, "values": tr.values,
+              "rewards": tr.rewards, "dones": tr.dones, "advantages": tr.advantages, "returns": tr.returns}
+    out = {k: v.index_select(1, sel).float().cpu().numpy() for k, v in planes.items()}
+    out.update({"params": tr.agent.flat_params, "exp_avg": tr.exp_avg, "exp_avg_sq": tr.exp_avg_sq, "loss_terms": tr.loss_terms,
+                "grad_norm": tr.grad_norm})
+    out = {k: (v.float().cpu().numpy() if torch.is_tensor(v) else v) for k, v in out.items()}
+    out["env_index"] = cols.astype(np.float64)
+    ep = tr.metrics(with_episode_log="arrays")["episode_log"]
+    ep = {k: np.asarray(ep[k], dtype=np.float64) for k in ("step", "env", "ret", "len")}
+    keep = np.isin(ep["env"], cols)
+    order = np.lexsort((ep["env"][keep], ep["step"][keep]))       # the device appends in completion order: sort by (step, env)
+    out.update({f"episode_{k}": v[keep][order] for k, v in ep.items()})
+    total = sum(v.nbytes for v in out.values())
+    assert total <= DUMP_BYTES, f"dump of {total} bytes exceeds {DUMP_BYTES}"
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), v)
+    return {"dir": out_dir, "arrays": sorted(out), "bytes": total, "envs": len(cols)}
+
+
 def _multi_gpu_checks(tr, nu, dev, world):
     """Driver-visible multi-GPU correctness (GPUTEST runs on one GPU): (1) every rank holds bit-identical parameters and Adam
     moments after the timed updates; (2) two more updates from the same state through the in-kernel peer all-reduce and
@@ -489,6 +527,7 @@ def run_b200(args):
     evs, l0 = _timed_updates(tr, nu, args.steps, flush, dist, dev)
     clocks = sampler.stop() if sampler else None      # last sample while the queued updates are still running
     dev_ms, _, _, launches = _finish_timed(tr, evs, l0, dist, dev)
+    dumped = _dump_outputs(tr, args.dump_outputs) if args.dump_outputs and rank == 0 else None
     steps_per_update = envs * T * world
     value = steps_per_update * args.steps / (dev_ms * 1e-3)
     graphed = tr._graph is not None
@@ -624,7 +663,7 @@ def run_b200(args):
         "gpu_launches": launches, "clocks": clocks, "roofline": roofline, "rooflines": rooflines, "cpu_baseline": cpu_baseline,
         "phases_ms_per_update": {k: v["total_ms"] / args.steps for k, v in phases.items()},
         "cuda_graph": graphed, "ms_per_step_eager_instrumented": inst_ms / args.steps,
-        "scaling_reference": scaling_ref, "extra_configs": extra, "fp32_path": fp32_path,
+        "scaling_reference": scaling_ref, "extra_configs": extra, "fp32_path": fp32_path, "dumped_outputs": dumped,
     }
     if world > 1:
         line.update(multi)
@@ -667,7 +706,14 @@ def main():
                     help="multi-GPU gradient exchange: in-kernel NVLink peer-memory all-reduce, or NCCL between kernels")
     ap.add_argument("--precision", default="auto", choices=["auto", "bf16", "fp32"],
                     help="update GEMMs: bf16 = tcgen05 tensor cores (bf16 operands, fp32 accumulate), fp32 = CUDA cores")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed updates, write what the last one computed (parameters, Adam moments, loss terms, rollout "
+                         "planes, advantages, returns, finished episodes) as DIR/<name>.npy, at most 64 MiB; rank 0 only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     if args.impl == "reference":
         run_reference(args)
     else:

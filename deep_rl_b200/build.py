@@ -80,8 +80,11 @@ def build(force: bool = False, verbose: bool = False) -> str:
 def build_locked() -> str:
     """What the import path calls: returns the library path, rebuilding first if it is missing or stale.  The check and the
     build run under an exclusive file lock (all ranks of a torchrun job import at once).  A stale library without a
-    compiler at hand (the GPU box always has one; a stripped deployment may not) is used as it is."""
+    compiler at hand (a stripped deployment may not have one) is used as it is.  An up-to-date library is returned without
+    opening the lock file, so that a read-only installation imports."""
     import fcntl
+    if not is_stale():
+        return SO
     os.makedirs(LIBDIR, exist_ok=True)
     with open(os.path.join(LIBDIR, ".build.lock"), "w") as lk:
         fcntl.flock(lk, fcntl.LOCK_EX)

@@ -122,9 +122,11 @@ def main():
             out[f"u{upd}_{k}"] = v
     for key in ("lr", "terms", "grad_pre", "norm", "params_after"):
         out[f"mb_{key}"] = np.stack([np.asarray(e[key]) for e in rec["mb"]])
+    # the 16 pre-clip gradients go to a file of their own, so that neither file is larger than 1 MB
     path = os.path.join(ROOT, "tests", "golden", "ref_ppo_seed1.npz")
+    np.savez_compressed(os.path.join(ROOT, "tests", "golden", "ref_ppo_seed1_grads.npz"), mb_grad_pre=out.pop("mb_grad_pre"))
     np.savez_compressed(path, **out)
-    print(f"wrote {path}: {len(eps)} episodes, adam calls {state['adam_calls']}, "
+    print(f"wrote {path} (+ _grads): {len(eps)} episodes, adam calls {state['adam_calls']}, "
           f"first/last-20 mean return {eps[:20, 1].mean():.1f} / {eps[-20:, 1].mean():.1f}")
     print({k: v.shape for k, v in out.items()})
 
