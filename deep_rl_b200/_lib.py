@@ -36,6 +36,10 @@ class RolloutBufT(C.Structure):
                 ("rew", C.c_void_p), ("done", C.c_void_p), ("logits", C.c_void_p)]
 
 
+class EvalTraceT(C.Structure):
+    _fields_ = [("state", C.c_void_p), ("obs", C.c_void_p), ("logits", C.c_void_p), ("act", C.c_void_p)]
+
+
 class CommT(C.Structure):
     _fields_ = [("world", C.c_int32), ("rank", C.c_int32), ("peer", C.c_void_p * 8), ("seq", C.c_uint32),
                 ("error_flag", C.c_void_p)]
@@ -69,6 +73,8 @@ SIGNATURES = {
     "drl_sample": (C.c_int, [f32p, C.c_int64, C.c_int32, C.c_uint64, C.c_uint32, C.c_uint64, i32p, f32p, C.c_void_p]),
     "drl_rollout": (C.c_int, [C.POINTER(EnvT), C.POINTER(NetT), f32p, C.c_int32, C.c_uint64, C.POINTER(RolloutBufT),
                               C.POINTER(EpLogT), C.c_uint32, C.c_void_p]),
+    "drl_evaluate": (C.c_int, [C.POINTER(EnvT), C.POINTER(NetT), f32p, C.c_int32, C.c_uint32, C.POINTER(EpLogT),
+                               C.POINTER(EvalTraceT), C.c_void_p]),
     "drl_gae": (C.c_int, [C.POINTER(RolloutBufT), C.POINTER(NetT), C.c_int32, C.c_int32, C.c_float, C.c_float, f32p,
                           f32p, f32p, C.c_void_p]),
     "drl_explained_variance": (C.c_int, [f32p, f32p, C.c_int64, f32p, C.c_void_p, C.c_size_t, C.c_void_p]),

@@ -34,6 +34,14 @@ import torch
 from . import _lib, dist as _dist
 from .agent import ActorCritic
 from .envs import VecEnv
+from .evaluate import EvalResult, evaluate as _evaluate
+
+EVAL_SEED_OFFSET = 0x9E3779B97F4A7C15     # default evaluation key = (cfg.seed + this) mod 2^64: never a training key
+
+
+def eval_seed(seed: int) -> int:
+    """The default evaluation key of a trainer keyed `seed`."""
+    return (int(seed) + EVAL_SEED_OFFSET) % (1 << 64)
 
 
 @dataclass
@@ -71,6 +79,8 @@ class PPOConfig:
                                      # matter -- else 1)
     cuda_graph: bool = True          # tcgen05 path: capture the launches of one update in a CUDA graph (counters live in a
                                      # device-resident drl_ctrl_t) and replay it; results are bit-identical to the eager path
+    eval_every: int = 0              # train(): greedy evaluation after every eval_every-th update (0 = off)
+    eval_episodes: int = 1024        # envs of that evaluation, one fresh episode each
 
     def resolved_update_precision(self) -> str:
         if self.update_precision == "auto":
@@ -554,13 +564,24 @@ class PPOTrainer:
                                                  _lib.stream_ptr()))
         return float(self._ev_out.item())
 
+    def evaluate(self, num_envs: int = 1024, episodes_per_env: int = 1, greedy: bool = True,
+                 seed: Optional[int] = None) -> EvalResult:
+        """Evaluate the current policy on `num_envs` fresh envs x `episodes_per_env` episodes (one drl_evaluate launch on
+        private envs and log; synchronises).  Touches no trainer state: training continues bit-identically.  The key
+        defaults to eval_seed(cfg.seed); rank r plays global env ids [r * num_envs, (r + 1) * num_envs), so ranks play
+        disjoint episodes -- pooling them across ranks (e.g. torch.distributed.all_gather of `returns`) is the caller's."""
+        return _evaluate(self.agent, self.cfg.env_id, num_envs, episodes_per_env, greedy,
+                         eval_seed(self.cfg.seed) if seed is None else seed, env_gid0=self.rank * int(num_envs))
+
 
 def train(cfg: PPOConfig, quiet: bool = False, rank: int = 0, world: int = 1) -> PPOTrainer:
-    """The training loop of the reference script; prints its `global_step=..., episodic_return=...` lines."""
+    """The training loop of the reference script; prints its `global_step=..., episodic_return=...` lines.  With
+    cfg.eval_every > 0, after every eval_every-th update a greedy evaluation over cfg.eval_episodes fresh episodes follows,
+    printed by rank 0 as `global_step=..., eval_return=<mean>±<std> (greedy, <n> episodes)` (rank 0's episodes)."""
     tr = PPOTrainer(cfg, rank=rank, world=world)
     nu = cfg.num_updates(world)
     per_vec_step = cfg.num_envs * world
-    for _ in range(nu):
+    for u in range(nu):
         tr.update(nu)
         m = tr.metrics()
         if not quiet and rank == 0:
@@ -570,6 +591,11 @@ def train(cfg: PPOConfig, quiet: bool = False, rank: int = 0, world: int = 1) ->
             elif m["episodes"]:
                 print(f"global_step={tr.global_step}, episodic_return={m['mean_return']:.2f} "
                       f"(mean of {m['episodes']} episodes)")
+        if cfg.eval_every > 0 and (u + 1) % cfg.eval_every == 0:
+            ev = tr.evaluate(num_envs=cfg.eval_episodes, episodes_per_env=1, greedy=True)
+            if not quiet and rank == 0:
+                print(f"global_step={tr.global_step}, eval_return={ev.mean_return:.2f}±{ev.std_return:.2f} "
+                      f"(greedy, {ev.episodes} episodes)")
     return tr
 
 
@@ -583,10 +609,13 @@ def main(argv=None) -> None:
     p.add_argument("--update-epochs", type=int, default=d.update_epochs)
     p.add_argument("--learning-rate", type=float, default=d.learning_rate)
     p.add_argument("--seed", type=int, default=d.seed)
+    p.add_argument("--eval-every", type=int, default=d.eval_every, help="greedy evaluation every N updates (0 = off)")
+    p.add_argument("--eval-episodes", type=int, default=d.eval_episodes)
     a = p.parse_args(argv)
     rank, world = _dist.init_from_env()
     cfg = PPOConfig(env_id=a.env_id, total_timesteps=a.total_timesteps, num_steps=a.num_steps, num_envs=a.num_envs,
-                    update_epochs=a.update_epochs, learning_rate=a.learning_rate, seed=a.seed)
+                    update_epochs=a.update_epochs, learning_rate=a.learning_rate, seed=a.seed, eval_every=a.eval_every,
+                    eval_episodes=a.eval_episodes)
     train(cfg, rank=rank, world=world)
     _dist.shutdown()
 

@@ -142,6 +142,25 @@ int drl_sample(const float* logits /*[n][A]*/, int64_t n, int32_t num_actions, u
 int drl_rollout(const drl_env_t* env, const drl_net_t* net, const float* packed, int32_t T, uint64_t step0,
                 const drl_rollout_buf_t* buf, const drl_ep_log_t* log, uint32_t flags, void* stream);
 
+/* ---- policy evaluation on fresh episodes: every env plays episodes_per_env = K whole episodes of the frozen policy in one
+ * launch (fp32 CUDA cores, hidden = 64 only).  Env n starts from the reset draw of drl_env_reset (env->seed is the evaluation
+ * key, env->state's contents are ignored) and takes steps t = 0, 1, ...: the action is the first index of the largest logit
+ * (DRL_EVAL_GREEDY) or drl_rollout's Philox draw with step index t; TimeLimit and auto-reset as drl_env_step(step = t).
+ * An env stops after its K-th finished episode, so the log receives exactly N * K entries {step, env, ret, len}; log is
+ * required, with cap >= N * K.  On return env->state / elapsed / ep_ret / ep_len hold the final state.
+ * trace (nullable, every plane nullable; tests): S = K * max_episode_steps rows; row t of env n holds the state the action of
+ * step t was chosen in, its observation, its logits and the action; act is 0xFF in the rows after the env's quota (the other
+ * planes are not written there). */
+#define DRL_EVAL_GREEDY 1u   /* flags: argmax action instead of the Philox sample */
+typedef struct {
+    double*  state;    /* [S][N][4] */
+    float*   obs;      /* [S][N][OP] */
+    float*   logits;   /* [S][N][A] */
+    uint8_t* act;      /* [S][N] */
+} drl_eval_trace_t;
+int drl_evaluate(const drl_env_t* env, const drl_net_t* net, const float* packed, int32_t episodes_per_env, uint32_t flags,
+                 const drl_ep_log_t* log, const drl_eval_trace_t* trace /* nullable */, void* stream);
+
 /* ---- graph-replayable variants: same kernels, counters read from *ctrl (device memory) ----
  * drl_ctrl_set computes the Adam scalars of the coming n_steps optimizer steps (same fp64 host arithmetic as drl_clip_adam) and
  * writes the whole block with one kernel launch. */
