@@ -75,6 +75,8 @@ SIGNATURES = {
                               C.POINTER(EpLogT), C.c_uint32, C.c_void_p]),
     "drl_evaluate": (C.c_int, [C.POINTER(EnvT), C.POINTER(NetT), f32p, C.c_int32, C.c_uint32, C.POINTER(EpLogT),
                                C.POINTER(EvalTraceT), C.c_void_p]),
+    "drl_evaluate_tc": (C.c_int, [C.POINTER(EnvT), C.POINTER(NetT), f32p, C.c_int32, C.c_uint32, C.POINTER(EpLogT),
+                                  C.POINTER(EvalTraceT), C.c_void_p]),
     "drl_gae": (C.c_int, [C.POINTER(RolloutBufT), C.POINTER(NetT), C.c_int32, C.c_int32, C.c_float, C.c_float, f32p,
                           f32p, f32p, C.c_void_p]),
     "drl_explained_variance": (C.c_int, [f32p, f32p, C.c_int64, f32p, C.c_void_p, C.c_size_t, C.c_void_p]),

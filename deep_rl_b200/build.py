@@ -18,7 +18,7 @@ LIBDIR = os.path.join(PKG, "lib")
 OBJDIR = os.path.join(PKG, "build")
 SO = os.path.join(LIBDIR, "libdrl_b200.so")
 
-SOURCES = ["abi_misc.cu", "env_ops.cu", "policy_ops.cu", "rollout.cu", "rollout_tc.cu", "gae_ops.cu", "update_ops.cu", "update_tc.cu", "umma_selftest.cu", "update256.cu", "rollout256.cu", "replay_ops.cu", "reinforce_ops.cu", "eval_ops.cu"]
+SOURCES = ["abi_misc.cu", "env_ops.cu", "policy_ops.cu", "rollout.cu", "rollout_tc.cu", "gae_ops.cu", "update_ops.cu", "update_tc.cu", "umma_selftest.cu", "update256.cu", "rollout256.cu", "replay_ops.cu", "reinforce_ops.cu", "eval_ops.cu", "eval256.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-fmad=false",
     "-Xcompiler", "-fPIC", "-Xptxas", "-v", "--expt-relaxed-constexpr",

@@ -168,6 +168,17 @@ __device__ __forceinline__ int sample_categorical(const float (&l)[A], float u, 
     return act;
 }
 
+// first index of the largest logit (the torch.argmax tie rule)
+template <int A>
+__device__ __forceinline__ int argmax_first(const float (&l)[A]) {
+    int best = 0;
+    float m = l[0];
+#pragma unroll
+    for (int a = 1; a < A; ++a)
+        if (l[a] > m) { m = l[a]; best = a; }
+    return best;
+}
+
 // The same draw with the log-probability left in two pieces, logp = diff - logf(sum): the fused rollout finishes it off the
 // critical path of the step.  Bit-identical to sample_categorical.
 template <int A>

@@ -10,6 +10,7 @@
 #include <cuda_bf16.h>
 
 #include "drl_common.cuh"
+#include "drl_tc_common.cuh"
 
 namespace drl {
 namespace h256 {
@@ -111,6 +112,148 @@ struct Grad256Args {
 };
 
 constexpr int STAGE_TILES = 4096;   // 128-sample tiles per net the staging buffers hold (524,288 samples per pair of launches)
+
+// ---- The actor's per-step forward pass on 128 envs, shared by rollout256_kernel (rollout256.cu) and evaluate256_kernel
+// (eval256.cu).  Both kernels run these phases and nothing else between observation and logits, so they compute
+// bit-identical logits for the same observation: a sampled evaluation replays what the training rollout would have done.
+// Threads: 16 compute warps (warp w: row quarter q = w & 3, column quarter j = w >> 2; thread row r = 32 q + lane) and the
+// MMA-issuer warp.  Named barriers (the issuer syncs, the 512 compute threads arrive):
+enum : uint32_t { RB_H1 = 1, RB_L1 = 5, RB_QUAD = 6 };     // h1 chunk c ready (1..4), operand tile ready, row-quarter exchange (6..9)
+constexpr uint32_t RB_ALL = TC_COMPUTE + 32;
+constexpr uint32_t AF_Z1 = 0, AF_Z2 = 256;                 // TMEM columns of z1 and z2
+
+template <int O, int A>
+struct RoSmem256 {
+    static constexpr int OFF_W2 = 0;
+    static constexpr int OFF_ACT = OFF_W2 + HH * HH * 2;
+    static constexpr int OFF_W1B = OFF_ACT + TILE_BYTES;
+    static constexpr int OFF_B2 = OFF_W1B + 2 * HH * 8 * 2;
+    static constexpr int OFF_W4 = OFF_B2 + HH * 4;
+    static constexpr int OFF_B4 = OFF_W4 + 3 * HH * 4;
+    static constexpr int OFF_OBS = OFF_B4 + 128;
+    static constexpr int OFF_XCH = OFF_OBS + 4096;
+    static constexpr int OFF_BAR = OFF_XCH + 4 * 3 * 128 * 4;
+    static constexpr int TOTAL = OFF_BAR + 64 + 1024;
+    static_assert(TOTAL <= 232448, "shared memory");
+};
+
+// S0 (owner threads): row r of the [obs_hi | 1 | obs_lo] operand tile of the K = 16 layer-1 GEMM
+template <int O, int OP>
+__device__ __forceinline__ void actor_l1_row(unsigned char* tOBS, int r, const float (&obs)[OP]) {
+    float o16[16];
+#pragma unroll
+    for (int i = 0; i < 16; ++i) o16[i] = 0.0f;
+#pragma unroll
+    for (int i = 0; i < O; ++i) {
+        const float hi = __bfloat162float(__float2bfloat16_rn(obs[i]));
+        o16[i] = hi;
+        o16[8 + i] = obs[i] - hi;
+    }
+    o16[O] = 1.0f;
+    umma::store_row_ns16(tOBS, TC_TILE, r, o16);
+    umma::fence_proxy_async();
+}
+
+// Issuer warp, one step: the layer-1 GEMM once the operand tile is complete (RB_L1), then the layer-2 GEMM (M128 N256 K256)
+// chunk by chunk as P0 completes the h1 chunks (RB_H1 + c).  Commits bars[1] after layer 1 and bars[2] after layer 2.
+__device__ __forceinline__ void actor_issue_step(uint32_t tmem, uint32_t aOBS, uint32_t aW1B, uint32_t aACT, uint32_t aW2, uint64_t* bars) {
+    constexpr uint32_t ID_L1 = umma::make_idesc(128, 256, false, false);
+    constexpr uint32_t ID_FWD = umma::make_idesc(128, 256, false, false);
+    named_bar_sync(RB_L1, RB_ALL);
+    umma::fence_after_sync();
+    if (umma::elect_one()) {
+        umma::mma(tmem + AF_Z1, umma::make_desc(aOBS, 2048, 128, umma::LAYOUT_NONE),
+                  umma::make_desc(aW1B, 4096, 128, umma::LAYOUT_NONE), ID_L1, 0u);
+        umma::commit(bars + 1);
+    }
+    __syncwarp();
+#pragma unroll 1
+    for (int c = 0; c < NCH; ++c) {
+        named_bar_sync(RB_H1 + c, RB_ALL);
+        umma::fence_after_sync();
+        if (umma::elect_one()) {
+#pragma unroll
+            for (int kb = 0; kb < 4; ++kb)
+                umma::mma(tmem + AF_Z2, umma::make_desc(aACT + c * SLOT_BYTES + kb * 32, 16, 1024, umma::LAYOUT_SW128),
+                          umma::make_desc(aW2 + c * 32768 + kb * 32, 16, 1024, umma::LAYOUT_SW128), ID_FWD, (c > 0 || kb > 0) ? 1u : 0u);
+            if (c == NCH - 1) umma::commit(bars + 2);
+        }
+        __syncwarp();
+    }
+}
+
+// P0 (all compute threads): wait for layer 1, h1 = tanh(z1) -> four bf16 K-chunks of the layer-2 A operand; each chunk is
+// released to the issuer as soon as it is written.  `parity` = phase of bars[1] (step & 1).
+__device__ __forceinline__ void actor_h1_chunks(uint32_t trow, unsigned char* tACT, uint32_t off0, uint32_t off1, int j, uint64_t* bars,
+                                                uint32_t parity) {
+    mbar_wait(bars + 1, parity);
+    umma::fence_after_sync();
+#pragma unroll 1
+    for (int c = 0; c < NCH; ++c) {
+        float z[16];
+        umma::ld16(trow + AF_Z1 + 64 * c + 16 * j, z);
+#pragma unroll
+        for (int x = 0; x < 16; ++x) z[x] = tanh_mufu(z[x]);
+        uint4 q0, q1;
+        q0.x = umma::pack_bf16(z[0], z[1]); q0.y = umma::pack_bf16(z[2], z[3]); q0.z = umma::pack_bf16(z[4], z[5]); q0.w = umma::pack_bf16(z[6], z[7]);
+        q1.x = umma::pack_bf16(z[8], z[9]); q1.y = umma::pack_bf16(z[10], z[11]); q1.z = umma::pack_bf16(z[12], z[13]); q1.w = umma::pack_bf16(z[14], z[15]);
+        *reinterpret_cast<uint4*>(tACT + c * SLOT_BYTES + off0) = q0;
+        *reinterpret_cast<uint4*>(tACT + c * SLOT_BYTES + off1) = q1;
+        umma::fence_proxy_async();
+        umma::fence_before_sync();
+        named_bar_arrive(RB_H1 + c, RB_ALL);
+    }
+}
+
+// P1 (all compute threads): wait for layer 2, h2 = tanh(z2 + b2) on this thread's 64 units, partial head sums -> xch
+// (the caller makes them visible to its row quarter with RB_QUAD + q).  `parity` = phase of bars[2] (step & 1).
+template <int A>
+__device__ __forceinline__ void actor_head_partials(uint32_t trow, const float* sB2, const float* sW4, float* xch, int j, int r,
+                                                    uint64_t* bars, uint32_t parity) {
+    mbar_wait(bars + 2, parity);
+    umma::fence_after_sync();
+    float ps[A];
+#pragma unroll
+    for (int a = 0; a < A; ++a) ps[a] = 0.0f;
+#pragma unroll 1
+    for (int c = 0; c < NCH; ++c) {
+        float z[16];
+        umma::ld16(trow + AF_Z2 + 64 * c + 16 * j, z);
+#pragma unroll
+        for (int e4 = 0; e4 < 4; ++e4) {
+            const float4 bb = *reinterpret_cast<const float4*>(sB2 + 64 * c + 16 * j + 4 * e4);
+            z[4 * e4 + 0] = tanh_mufu(z[4 * e4 + 0] + bb.x);
+            z[4 * e4 + 1] = tanh_mufu(z[4 * e4 + 1] + bb.y);
+            z[4 * e4 + 2] = tanh_mufu(z[4 * e4 + 2] + bb.z);
+            z[4 * e4 + 3] = tanh_mufu(z[4 * e4 + 3] + bb.w);
+        }
+#pragma unroll
+        for (int a = 0; a < A; ++a) {
+            const float* w = sW4 + a * HH + 64 * c + 16 * j;
+            float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f;
+#pragma unroll
+            for (int e4 = 0; e4 < 4; ++e4) {
+                const float4 ww = *reinterpret_cast<const float4*>(w + 4 * e4);
+                s0 = fmaf(z[4 * e4 + 0], ww.x, s0);
+                s1 = fmaf(z[4 * e4 + 1], ww.y, s1);
+                s2 = fmaf(z[4 * e4 + 2], ww.z, s2);
+                s3 = fmaf(z[4 * e4 + 3], ww.w, s3);
+            }
+            ps[a] += (s0 + s1) + (s2 + s3);
+        }
+    }
+#pragma unroll
+    for (int a = 0; a < A; ++a) xch[(j * 3 + a) * TC_TILE + r] = ps[a];
+}
+
+// S3 (owner threads, after the exchange barrier): the logits of row r, summed in a fixed order over the four column quarters
+template <int A>
+__device__ __forceinline__ void actor_logits(const float* xch, const float* sB4, int r, float (&l)[A]) {
+#pragma unroll
+    for (int a = 0; a < A; ++a)
+        l[a] = ((xch[(0 * 3 + a) * TC_TILE + r] + xch[(1 * 3 + a) * TC_TILE + r]) +
+                (xch[(2 * 3 + a) * TC_TILE + r] + xch[(3 * 3 + a) * TC_TILE + r])) + sB4[a];
+}
 
 }  // namespace h256
 }  // namespace drl

@@ -19,17 +19,6 @@ int pick_envs_per_warp(int N);     // rollout.cu: DRL_ROLLOUT_EPW forces the eva
 
 constexpr int EV_WARPS = 4;
 
-// first index of the largest logit (the torch.argmax tie rule)
-template <int A>
-__device__ __forceinline__ int argmax_first(const float (&l)[A]) {
-    int best = 0;
-    float m = l[0];
-#pragma unroll
-    for (int a = 1; a < A; ++a)
-        if (l[a] > m) { m = l[a]; best = a; }
-    return best;
-}
-
 template <int KIND, int SUB, int TL>
 __global__ void __launch_bounds__(EV_WARPS * 32) evaluate_kernel(drl_env_t env, const float* __restrict__ packed, int episodes_per_env,
                                                                  int S, bool greedy, drl_ep_log_t log, drl_eval_trace_t tr) {

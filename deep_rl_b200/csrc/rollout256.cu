@@ -6,6 +6,8 @@
 //        chunk behind them
 //   P1   h2 = tanh(z2 + b2), partial head sums (64 units per thread), exchange among the four threads of a row
 //   S3   owners: logits, Philox inverse-CDF sample, log-prob, fp64 env step with auto-reset and episode statistics, stores
+// The actor phases (S0's operand tile, P0, P1, the logits sum and the issuer's MMAs) live in drl_h256.cuh, shared with
+// evaluate256_kernel (eval256.cu), so that an evaluation computes the same logits as the rollout bit for bit.
 // The critic is not needed to advance the environments: values V(obs[t]) for all (T+1) x N stored observations are computed
 // afterwards by one batched forward pass of the critic (mlp256_kernel in forward mode, update256.cu) -- a plain GEMM-shaped
 // launch instead of a second 128 KB weight image per step.
@@ -22,24 +24,6 @@ namespace h256 {
 
 int launch_forward256(const drl_net_t* net, const float* packed, const float* obs, int64_t n, float* logits, float* value,
                       int only_net, cudaStream_t st);
-
-enum : uint32_t { RB_H1 = 1, RB_L1 = 5, RB_QUAD = 6 };
-constexpr uint32_t RB_ALL = TC_COMPUTE + 32;
-
-template <int O, int A>
-struct RoSmem256 {
-    static constexpr int OFF_W2 = 0;
-    static constexpr int OFF_ACT = OFF_W2 + HH * HH * 2;
-    static constexpr int OFF_W1B = OFF_ACT + TILE_BYTES;
-    static constexpr int OFF_B2 = OFF_W1B + 2 * HH * 8 * 2;
-    static constexpr int OFF_W4 = OFF_B2 + HH * 4;
-    static constexpr int OFF_B4 = OFF_W4 + 3 * HH * 4;
-    static constexpr int OFF_OBS = OFF_B4 + 128;
-    static constexpr int OFF_XCH = OFF_OBS + 4096;
-    static constexpr int OFF_BAR = OFF_XCH + 4 * 3 * 128 * 4;
-    static constexpr int TOTAL = OFF_BAR + 64 + 1024;
-    static_assert(TOTAL <= 232448, "shared memory");
-};
 
 template <int KIND>
 __global__ void __launch_bounds__(TC_THREADS, 1) rollout256_kernel(drl_env_t env, const float* __restrict__ packed, int T, uint64_t step0,
@@ -84,35 +68,10 @@ __global__ void __launch_bounds__(TC_THREADS, 1) rollout256_kernel(drl_env_t env
     }
     const uint32_t tmem = *slot;
     mbar_wait(bars, 0);
-    constexpr uint32_t C_Z1 = 0, C_Z2 = 256;
 
     if (is_mma_warp) {
         const uint32_t aW2 = smem_u32(tW2), aACT = smem_u32(tACT), aW1B = smem_u32(tW1B), aOBS = smem_u32(tOBS);
-        constexpr uint32_t ID_L1 = umma::make_idesc(128, 256, false, false);
-        constexpr uint32_t ID_FWD = umma::make_idesc(128, 256, false, false);
-        for (int t = 0; t < T; ++t) {
-            named_bar_sync(RB_L1, RB_ALL);
-            umma::fence_after_sync();
-            if (umma::elect_one()) {
-                umma::mma(tmem + C_Z1, umma::make_desc(aOBS, 2048, 128, umma::LAYOUT_NONE),
-                          umma::make_desc(aW1B, 4096, 128, umma::LAYOUT_NONE), ID_L1, 0u);
-                umma::commit(bars + 1);
-            }
-            __syncwarp();
-#pragma unroll 1
-            for (int c = 0; c < NCH; ++c) {
-                named_bar_sync(RB_H1 + c, RB_ALL);
-                umma::fence_after_sync();
-                if (umma::elect_one()) {
-#pragma unroll
-                    for (int kb = 0; kb < 4; ++kb)
-                        umma::mma(tmem + C_Z2, umma::make_desc(aACT + c * SLOT_BYTES + kb * 32, 16, 1024, umma::LAYOUT_SW128),
-                                  umma::make_desc(aW2 + c * 32768 + kb * 32, 16, 1024, umma::LAYOUT_SW128), ID_FWD, (c > 0 || kb > 0) ? 1u : 0u);
-                    if (c == NCH - 1) umma::commit(bars + 2);
-                }
-                __syncwarp();
-            }
-        }
+        for (int t = 0; t < T; ++t) actor_issue_step(tmem, aOBS, aW1B, aACT, aW2, bars);
         umma::fence_before_sync();
         __syncthreads();
         umma::tmem_dealloc(tmem, 512);
@@ -145,81 +104,17 @@ __global__ void __launch_bounds__(TC_THREADS, 1) rollout256_kernel(drl_env_t env
 #pragma unroll
                 for (int qq = 0; qq < OP / 4; ++qq) o4[qq] = make_float4(obs[4 * qq], obs[4 * qq + 1], obs[4 * qq + 2], obs[4 * qq + 3]);
             }
-            if (t < T) {
-                float o16[16];
-#pragma unroll
-                for (int i = 0; i < 16; ++i) o16[i] = 0.0f;
-#pragma unroll
-                for (int i = 0; i < O; ++i) {
-                    const float hi = __bfloat162float(__float2bfloat16_rn(obs[i]));
-                    o16[i] = hi;
-                    o16[8 + i] = obs[i] - hi;
-                }
-                o16[O] = 1.0f;
-                umma::store_row_ns16(tOBS, TC_TILE, r, o16);
-                umma::fence_proxy_async();
-            }
+            if (t < T) actor_l1_row<O, OP>(tOBS, r, obs);
         }
         if (t == T) break;            // the last observation needs no action (its value comes from the critic pass)
         umma::fence_before_sync();
         named_bar_arrive(RB_L1, RB_ALL);
 
         // ---- P0: h1 chunks ----
-        mbar_wait(bars + 1, (uint32_t)t & 1u);
-        umma::fence_after_sync();
-#pragma unroll 1
-        for (int c = 0; c < NCH; ++c) {
-            float z[16];
-            umma::ld16(trow + C_Z1 + 64 * c + 16 * j, z);
-#pragma unroll
-            for (int x = 0; x < 16; ++x) z[x] = tanh_mufu(z[x]);
-            uint4 q0, q1;
-            q0.x = umma::pack_bf16(z[0], z[1]); q0.y = umma::pack_bf16(z[2], z[3]); q0.z = umma::pack_bf16(z[4], z[5]); q0.w = umma::pack_bf16(z[6], z[7]);
-            q1.x = umma::pack_bf16(z[8], z[9]); q1.y = umma::pack_bf16(z[10], z[11]); q1.z = umma::pack_bf16(z[12], z[13]); q1.w = umma::pack_bf16(z[14], z[15]);
-            *reinterpret_cast<uint4*>(tACT + c * SLOT_BYTES + off0) = q0;
-            *reinterpret_cast<uint4*>(tACT + c * SLOT_BYTES + off1) = q1;
-            umma::fence_proxy_async();
-            umma::fence_before_sync();
-            named_bar_arrive(RB_H1 + c, RB_ALL);
-        }
+        actor_h1_chunks(trow, tACT, off0, off1, j, bars, (uint32_t)t & 1u);
 
         // ---- P1: layer-2 epilogue and partial head sums ----
-        mbar_wait(bars + 2, (uint32_t)t & 1u);
-        umma::fence_after_sync();
-        {
-            float ps[A];
-#pragma unroll
-            for (int a = 0; a < A; ++a) ps[a] = 0.0f;
-#pragma unroll 1
-            for (int c = 0; c < NCH; ++c) {
-                float z[16];
-                umma::ld16(trow + C_Z2 + 64 * c + 16 * j, z);
-#pragma unroll
-                for (int e4 = 0; e4 < 4; ++e4) {
-                    const float4 bb = *reinterpret_cast<const float4*>(sB2 + 64 * c + 16 * j + 4 * e4);
-                    z[4 * e4 + 0] = tanh_mufu(z[4 * e4 + 0] + bb.x);
-                    z[4 * e4 + 1] = tanh_mufu(z[4 * e4 + 1] + bb.y);
-                    z[4 * e4 + 2] = tanh_mufu(z[4 * e4 + 2] + bb.z);
-                    z[4 * e4 + 3] = tanh_mufu(z[4 * e4 + 3] + bb.w);
-                }
-#pragma unroll
-                for (int a = 0; a < A; ++a) {
-                    const float* w = sW4 + a * HH + 64 * c + 16 * j;
-                    float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f;
-#pragma unroll
-                    for (int e4 = 0; e4 < 4; ++e4) {
-                        const float4 ww = *reinterpret_cast<const float4*>(w + 4 * e4);
-                        s0 = fmaf(z[4 * e4 + 0], ww.x, s0);
-                        s1 = fmaf(z[4 * e4 + 1], ww.y, s1);
-                        s2 = fmaf(z[4 * e4 + 2], ww.z, s2);
-                        s3 = fmaf(z[4 * e4 + 3], ww.w, s3);
-                    }
-                    ps[a] += (s0 + s1) + (s2 + s3);
-                }
-            }
-#pragma unroll
-            for (int a = 0; a < A; ++a) xch[(j * 3 + a) * TC_TILE + r] = ps[a];
-        }
+        actor_head_partials<A>(trow, sB2, sW4, xch, j, r, bars, (uint32_t)t & 1u);
         umma::fence_before_sync();
         named_bar_sync(RB_QUAD + q, 128);
 
@@ -227,10 +122,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) rollout256_kernel(drl_env_t env
         if (own) {
             const size_t i0 = (size_t)t * N + n;
             float l[A];
-#pragma unroll
-            for (int a = 0; a < A; ++a)
-                l[a] = ((xch[(0 * 3 + a) * TC_TILE + r] + xch[(1 * 3 + a) * TC_TILE + r]) +
-                        (xch[(2 * 3 + a) * TC_TILE + r] + xch[(3 * 3 + a) * TC_TILE + r])) + sB4[a];
+            actor_logits<A>(xch, sB4, r, l);
             if (buf.logits != nullptr) {
 #pragma unroll
                 for (int a = 0; a < A; ++a) buf.logits[i0 * A + a] = l[a];

@@ -1,4 +1,5 @@
-"""Policy evaluation on fresh episodes: N envs x K whole episodes of a frozen policy in ONE kernel launch (drl_evaluate).
+"""Policy evaluation on fresh episodes: N envs x K whole episodes of a frozen policy in ONE kernel launch (drl_evaluate for
+64-wide nets, fp32 CUDA cores; drl_evaluate_tc for 256-wide nets, tcgen05 with the training rollout's bf16 numerics).
 
 The counterpart of CleanRL's eval scripts and SB3's `evaluate_policy`: unlike `PPOTrainer.metrics()["mean_return"]` (the
 training episodes that happened to finish inside one rollout window, produced by several successive policies, always
@@ -44,8 +45,8 @@ class EvalResult:
 
 def evaluate(agent, env_id: str, num_envs: int, episodes_per_env: int = 1, greedy: bool = True, seed: int = 0,
              env_gid0: int = 0, trace: bool = False) -> EvalResult:
-    """Play `episodes_per_env` episodes on each of `num_envs` fresh envs with `agent`'s current parameters (fp32 forward,
-    hidden = 64).  `seed` is the evaluation key of the env resets and of the sampled actions; `env_gid0` the global id of
+    """Play `episodes_per_env` episodes on each of `num_envs` fresh envs with `agent`'s current parameters: fp32 forward for
+    hidden = 64 (drl_evaluate), the tensor-core forward of the training rollout for hidden = 256 (drl_evaluate_tc).  `seed` is the evaluation key of the env resets and of the sampled actions; `env_gid0` the global id of
     env 0.  Synchronises the current stream once, to read the episode log.  `trace=True` also returns the per-step planes
     (tests; S * N * (32 + 4 * OP + 4 * A + 1) bytes)."""
     _lib.require_cuda()
@@ -64,12 +65,13 @@ def evaluate(agent, env_id: str, num_envs: int, episodes_per_env: int = 1, greed
                "logits": torch.zeros((S, N, env.num_actions), dtype=torch.float32, device=dev),
                "act": torch.zeros((S, N), dtype=torch.uint8, device=dev)}
         tr = _lib.EvalTraceT(*(out[k].data_ptr() for k in ("state", "obs", "logits", "act")))
-    _lib.check(env.L.drl_evaluate(C.byref(env.struct), C.byref(agent.net), agent.packed.data_ptr(), K,
-                                  DRL_EVAL_GREEDY if greedy else 0, C.byref(env.log.struct),
-                                  C.byref(tr) if tr is not None else None, _lib.stream_ptr()))
+    name = "drl_evaluate_tc" if agent.hidden == 256 else "drl_evaluate"
+    _lib.check(getattr(env.L, name)(C.byref(env.struct), C.byref(agent.net), agent.packed.data_ptr(), K,
+                                    DRL_EVAL_GREEDY if greedy else 0, C.byref(env.log.struct),
+                                    C.byref(tr) if tr is not None else None, _lib.stream_ptr()))
     n, _, _, e = env.log.drain_arrays()
     if n != N * K:
-        raise _lib.DrlError(f"drl_evaluate logged {n} episodes, expected {N * K}")
+        raise _lib.DrlError(f"{name} logged {n} episodes, expected {N * K}")
     order = np.lexsort((e["step"], e["env"]))          # by env, then by the step the episode ended at
     returns = np.ascontiguousarray(e["ret"][order]).reshape(N, K).copy()
     lengths = np.ascontiguousarray(e["len"][order]).reshape(N, K).astype(np.int32)

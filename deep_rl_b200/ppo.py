@@ -566,8 +566,9 @@ class PPOTrainer:
 
     def evaluate(self, num_envs: int = 1024, episodes_per_env: int = 1, greedy: bool = True,
                  seed: Optional[int] = None) -> EvalResult:
-        """Evaluate the current policy on `num_envs` fresh envs x `episodes_per_env` episodes (one drl_evaluate launch on
-        private envs and log; synchronises).  Touches no trainer state: training continues bit-identically.  The key
+        """Evaluate the current policy on `num_envs` fresh envs x `episodes_per_env` episodes (one drl_evaluate launch, or
+        drl_evaluate_tc for a 256-wide net, on private envs and log; synchronises).  Touches no trainer state: training
+        continues bit-identically.  The key
         defaults to eval_seed(cfg.seed); rank r plays global env ids [r * num_envs, (r + 1) * num_envs), so ranks play
         disjoint episodes -- pooling them across ranks (e.g. torch.distributed.all_gather of `returns`) is the caller's."""
         return _evaluate(self.agent, self.cfg.env_id, num_envs, episodes_per_env, greedy,
@@ -611,11 +612,12 @@ def main(argv=None) -> None:
     p.add_argument("--seed", type=int, default=d.seed)
     p.add_argument("--eval-every", type=int, default=d.eval_every, help="greedy evaluation every N updates (0 = off)")
     p.add_argument("--eval-episodes", type=int, default=d.eval_episodes)
+    p.add_argument("--hidden", type=int, default=d.hidden, choices=(64, 256), help="width of both hidden layers")
     a = p.parse_args(argv)
     rank, world = _dist.init_from_env()
     cfg = PPOConfig(env_id=a.env_id, total_timesteps=a.total_timesteps, num_steps=a.num_steps, num_envs=a.num_envs,
                     update_epochs=a.update_epochs, learning_rate=a.learning_rate, seed=a.seed, eval_every=a.eval_every,
-                    eval_episodes=a.eval_episodes)
+                    eval_episodes=a.eval_episodes, hidden=a.hidden)
     train(cfg, rank=rank, world=world)
     _dist.shutdown()
 

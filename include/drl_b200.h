@@ -143,7 +143,7 @@ int drl_rollout(const drl_env_t* env, const drl_net_t* net, const float* packed,
                 const drl_rollout_buf_t* buf, const drl_ep_log_t* log, uint32_t flags, void* stream);
 
 /* ---- policy evaluation on fresh episodes: every env plays episodes_per_env = K whole episodes of the frozen policy in one
- * launch (fp32 CUDA cores, hidden = 64 only).  Env n starts from the reset draw of drl_env_reset (env->seed is the evaluation
+ * launch (fp32 CUDA cores, hidden = 64 only; drl_evaluate_tc below for hidden = 256).  Env n starts from the reset draw of drl_env_reset (env->seed is the evaluation
  * key, env->state's contents are ignored) and takes steps t = 0, 1, ...: the action is the first index of the largest logit
  * (DRL_EVAL_GREEDY) or drl_rollout's Philox draw with step index t; TimeLimit and auto-reset as drl_env_step(step = t).
  * An env stops after its K-th finished episode, so the log receives exactly N * K entries {step, env, ret, len}; log is
@@ -160,6 +160,13 @@ typedef struct {
 } drl_eval_trace_t;
 int drl_evaluate(const drl_env_t* env, const drl_net_t* net, const float* packed, int32_t episodes_per_env, uint32_t flags,
                  const drl_ep_log_t* log, const drl_eval_trace_t* trace /* nullable */, void* stream);
+/* The same evaluation -- arguments, validation, streams, log and trace -- on tcgen05 with the numerics of drl_rollout's
+ * DRL_ROLLOUT_TENSOR_CORES path (bf16 operands, fp32 accumulation, tanh.approx), for hidden = 256 only: one CTA steps 128
+ * envs and leaves when all of them have played their K episodes.  The logits of an observation are bit-identical to those
+ * drl_rollout computes for it, so a sampled evaluation replays the training rollout from the same state and keys.
+ * hidden = 64 returns DRL_ERR_UNSUPPORTED (use drl_evaluate), any other width DRL_ERR_ARG. */
+int drl_evaluate_tc(const drl_env_t* env, const drl_net_t* net, const float* packed, int32_t episodes_per_env, uint32_t flags,
+                    const drl_ep_log_t* log, const drl_eval_trace_t* trace /* nullable */, void* stream);
 
 /* ---- graph-replayable variants: same kernels, counters read from *ctrl (device memory) ----
  * drl_ctrl_set computes the Adam scalars of the coming n_steps optimizer steps (same fp64 host arithmetic as drl_clip_adam) and
