@@ -10,6 +10,7 @@
 // PPO path's (drl_env.cuh); the dropout mask of (env, step) is 128 Philox uniforms (one block per lane, TAG_DROPOUT), regenerated
 // in the backward pass instead of being stored.
 #include "drl_env.cuh"
+#include "drl_update.cuh"
 
 namespace drl {
 
@@ -224,10 +225,7 @@ __global__ void __launch_bounds__(256) adam_step_kernel(float* __restrict__ para
     if (i >= n) return;
     const float g = grad[i];
     float mi = m[i], vi = v[i], p = params[i];
-    mi = mi + om_beta1 * (g - mi);
-    vi = vi * beta2 + (om_beta2 * g) * g;
-    const float denom = sqrtf(vi) / bc2_sqrt + eps;
-    p = p + (neg_step_size * mi) / denom;
+    adam_apply(g, mi, vi, p, om_beta1, beta2, om_beta2, eps, neg_step_size, bc2_sqrt);
     m[i] = mi; v[i] = vi; params[i] = p;
 }
 
@@ -271,9 +269,9 @@ int drl_adam_step(float* params, const float* grad, float* exp_avg, float* exp_a
                   double beta2, double eps, void* stream) {
     DRL_REQUIRE(params && grad && exp_avg && exp_avg_sq, "drl_adam_step: NULL pointer");
     DRL_REQUIRE(n > 0 && step >= 1, "drl_adam_step: n=%lld step=%lld", (long long)n, (long long)step);
-    const double bc1 = 1.0 - pow(beta1, (double)step), bc2 = 1.0 - pow(beta2, (double)step);
+    const AdamScalars s = adam_scalars(step, lr, beta1, beta2);
     adam_step_kernel<<<(unsigned)((n + 255) / 256), 256, 0, as_stream(stream)>>>(params, grad, exp_avg, exp_avg_sq, n, (float)beta2, (float)(1.0 - beta1),
-                                                                              (float)(1.0 - beta2), (float)eps, (float)(-(lr / bc1)), (float)sqrt(bc2));
+                                                                              (float)(1.0 - beta2), (float)eps, s.neg_step_size, s.bc2_sqrt);
     DRL_LAUNCH_CHECK("adam_step_kernel");
     return DRL_OK;
 }

@@ -793,53 +793,6 @@ __global__ void __launch_bounds__(B_BLOCK, 1) dw2_gemm256_kernel(const unsigned 
     if (warp == 2) umma::tmem_dealloc(tmem, 512);
 }
 
-// Fixed-order fold of the per-CTA partial rows.  Parameter p of the actor is summed over the even rows, of the critic over the odd
-// rows (the other rows never wrote it).  blockDim = (32, 8): thread (x, y) folds rows first + 2 (y + 8 k), then the 8 slices are
-// folded through shared memory in slice order -- the association of grad_reduce_kernel (update_ops.cu).
-__global__ void __launch_bounds__(256) grad_reduce256_kernel(const float* __restrict__ grad_part, const float* __restrict__ loss_part,
-                                                              int nrows, int ppad, int P, int c_actor, uint32_t mb_count, float ent_coef,
-                                                              float vf_coef, float* __restrict__ grad_out, float* __restrict__ loss_terms_out) {
-    __shared__ float sh[8][33];
-    const int p = blockIdx.x * 32 + threadIdx.x;
-    float s = 0.0f;
-    if (p < P) {
-        const int first = p >= c_actor ? 1 : 0;
-        float a0 = 0.f, a1 = 0.f, a2 = 0.f, a3 = 0.f;
-        int c = first + 2 * threadIdx.y;
-        for (; c + 48 < nrows; c += 64) {
-            const float v0 = __ldcg(grad_part + (size_t)c * ppad + p);
-            const float v1 = __ldcg(grad_part + (size_t)(c + 16) * ppad + p);
-            const float v2 = __ldcg(grad_part + (size_t)(c + 32) * ppad + p);
-            const float v3 = __ldcg(grad_part + (size_t)(c + 48) * ppad + p);
-            a0 += v0; a1 += v1; a2 += v2; a3 += v3;
-        }
-        for (; c < nrows; c += 16) a0 += __ldcg(grad_part + (size_t)c * ppad + p);
-        s = (a0 + a1) + (a2 + a3);
-    }
-    sh[threadIdx.y][threadIdx.x] = s;
-    __syncthreads();
-    if (threadIdx.y == 0 && p < P) {
-        float t = sh[0][threadIdx.x];
-#pragma unroll
-        for (int y = 1; y < 8; ++y) t += sh[y][threadIdx.x];
-        grad_out[p] = t;
-    }
-    if (blockIdx.x == 0 && threadIdx.y == 1 && threadIdx.x < 5 && loss_terms_out != nullptr) {
-        float t = 0.f;
-        for (int c = 0; c < nrows; ++c) t += __ldcg(loss_part + c * LOSS_TERMS + threadIdx.x);
-        const float inv = 1.0f / (float)mb_count;
-        const float t0 = __shfl_sync(0x1fu, t, 0), t1 = __shfl_sync(0x1fu, t, 1), t2 = __shfl_sync(0x1fu, t, 2);
-        const float t3 = __shfl_sync(0x1fu, t, 3), t4 = __shfl_sync(0x1fu, t, 4);
-        if (threadIdx.x == 0) {
-            const float pg = t0 * inv, vl = 0.5f * t1 * inv, en = t2 * inv;
-            loss_terms_out[0] = pg - ent_coef * en + vl * vf_coef;
-            loss_terms_out[1] = pg; loss_terms_out[2] = vl; loss_terms_out[3] = en;
-            loss_terms_out[4] = t3 * inv; loss_terms_out[5] = t4 * inv;
-            loss_terms_out[6] = 0.0f; loss_terms_out[7] = 0.0f;
-        }
-    }
-}
-
 template <int O, int A, int OP, int RW>
 static int launch_grad256_t(const GradArgs& g0, int P, float* grad_out, float* loss_terms_out, void* workspace, cudaStream_t st) {
     const WorkspaceLayout w = workspace_layout(P, HH);
@@ -874,10 +827,7 @@ static int launch_grad256_t(const GradArgs& g0, int P, float* grad_out, float* l
     // rows critic entries, so each parameter is folded over the rows of its own net only
     const uint32_t first_tiles = ((g0.mb_count < chunk ? g0.mb_count : chunk) + TC_TILE - 1) / TC_TILE;
     const int active = (int)(2 * first_tiles < (uint32_t)grid ? 2 * first_tiles : (uint32_t)grid);
-    grad_reduce256_kernel<<<(P + 31) / 32, dim3(32, 8), 0, st>>>(g0.grad_part, g0.loss_part, active, g0.ppad, P, Packed256<O, A>::C_ACTOR,
-                                                              g0.mb_count, g0.ent_coef, g0.vf_coef, grad_out, loss_terms_out);
-    DRL_LAUNCH_CHECK("grad_reduce256_kernel");
-    return DRL_OK;
+    return launch_grad_reduce(g0, active, P, 2, Packed256<O, A>::C_ACTOR, grad_out, loss_terms_out, st);
 }
 
 int launch_grad256(const drl_net_t* net, const GradArgs& g, int P, float* grad_out, float* loss_terms_out, void* workspace,

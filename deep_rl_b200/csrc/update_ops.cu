@@ -354,29 +354,29 @@ __global__ void __launch_bounds__(GT, 1) ppo_grad_kernel(GradArgs g) {
     }
 }
 
-// Sum the per-CTA partials in a fixed order (deterministic) and finish the loss terms.  blockDim = (32, 8):
-// thread (x, y) folds partials y, y+8, ... of parameter p with independent loads in flight, then the 8
-// slices are folded through shared memory in slice order.
+// Lanes 0-4 of one warp each fold one loss term over the `nrows` per-CTA partials in row order, lane 0 then stores the
+// LOSS_TERMS row.  The five shuffles are written out: as an unrolled loop they lead nvcc to unroll the fold loop 4x, not 16x.
+__device__ __forceinline__ void fold_loss_terms(const float* __restrict__ loss_part, int nrows, uint32_t mb_count, float ent_coef,
+                                                float vf_coef, float* __restrict__ loss_terms_out) {
+    float t = 0.f;
+    for (int c = 0; c < nrows; ++c) t += __ldcg(loss_part + c * LOSS_TERMS + threadIdx.x);
+    const float sums[5] = {__shfl_sync(0x1fu, t, 0), __shfl_sync(0x1fu, t, 1), __shfl_sync(0x1fu, t, 2), __shfl_sync(0x1fu, t, 3),
+                           __shfl_sync(0x1fu, t, 4)};
+    if (threadIdx.x == 0) store_loss_terms(loss_terms_out, sums, mb_count, ent_coef, vf_coef);
+}
+
+// Sum the per-CTA partials in a fixed order (deterministic) and finish the loss terms.  blockDim = (32, 8): thread (x, y)
+// folds slice y of parameter p's rows (fold_partials) with independent loads in flight, then the 8 slices are added through
+// shared memory in slice order.  Row selection (STRIDE, critic0): launch_grad_reduce.  The stride is a template parameter:
+// with a constant trip-count divisor the compiler unrolls the fold and keeps more loads in flight.
+template <int STRIDE>
 __global__ void __launch_bounds__(256) grad_reduce_kernel(const float* __restrict__ grad_part, const float* __restrict__ loss_part,
-                                                           int nparts, int ppad, int P, uint32_t mb_count, float ent_coef,
-                                                           float vf_coef, float* __restrict__ grad_out,
-                                                           float* __restrict__ loss_terms_out) {
+                                                           int nrows, int ppad, int P, int critic0, uint32_t mb_count, float ent_coef,
+                                                           float vf_coef, float* __restrict__ grad_out, float* __restrict__ loss_terms_out) {
     __shared__ float sh[8][33];
     const int p = blockIdx.x * 32 + threadIdx.x;
     float s = 0.0f;
-    if (p < P) {
-        float a0 = 0.f, a1 = 0.f, a2 = 0.f, a3 = 0.f;
-        int c = threadIdx.y;
-        for (; c + 24 < nparts; c += 32) {
-            const float v0 = __ldcg(grad_part + (size_t)c * ppad + p);
-            const float v1 = __ldcg(grad_part + (size_t)(c + 8) * ppad + p);
-            const float v2 = __ldcg(grad_part + (size_t)(c + 16) * ppad + p);
-            const float v3 = __ldcg(grad_part + (size_t)(c + 24) * ppad + p);
-            a0 += v0; a1 += v1; a2 += v2; a3 += v3;
-        }
-        for (; c < nparts; c += 8) a0 += __ldcg(grad_part + (size_t)c * ppad + p);
-        s = (a0 + a1) + (a2 + a3);
-    }
+    if (p < P) s = fold_partials(grad_part, ppad, p, (p >= critic0 ? 1 : 0) + STRIDE * threadIdx.y, STRIDE, nrows);
     sh[threadIdx.y][threadIdx.x] = s;
     __syncthreads();
     if (threadIdx.y == 0 && p < P) {
@@ -385,25 +385,8 @@ __global__ void __launch_bounds__(256) grad_reduce_kernel(const float* __restric
         for (int y = 1; y < 8; ++y) t += sh[y][threadIdx.x];
         grad_out[p] = t;
     }
-    if (blockIdx.x == 0 && threadIdx.y == 1 && threadIdx.x < 5 && loss_terms_out != nullptr) {
-        // lanes 0-4 of warp 1 each fold one loss term over the CTAs, lane 0 then finishes the terms
-        float t = 0.f;
-        for (int c = 0; c < nparts; ++c) t += __ldcg(loss_part + c * LOSS_TERMS + threadIdx.x);
-        const float inv = 1.0f / (float)mb_count;
-        const float t0 = __shfl_sync(0x1fu, t, 0), t1 = __shfl_sync(0x1fu, t, 1), t2 = __shfl_sync(0x1fu, t, 2);
-        const float t3 = __shfl_sync(0x1fu, t, 3), t4 = __shfl_sync(0x1fu, t, 4);
-        if (threadIdx.x == 0) {
-            const float pg = t0 * inv, vl = 0.5f * t1 * inv, en = t2 * inv;
-            loss_terms_out[0] = pg - ent_coef * en + vl * vf_coef;
-            loss_terms_out[1] = pg;
-            loss_terms_out[2] = vl;
-            loss_terms_out[3] = en;
-            loss_terms_out[4] = t3 * inv;
-            loss_terms_out[5] = t4 * inv;
-            loss_terms_out[6] = 0.0f;
-            loss_terms_out[7] = 0.0f;
-        }
-    }
+    if (blockIdx.x == 0 && threadIdx.y == 1 && threadIdx.x < 5 && loss_terms_out != nullptr)
+        fold_loss_terms(loss_part, nrows, mb_count, ent_coef, vf_coef, loss_terms_out);
 }
 
 // clip_grad_norm_ + Adam.  Every CTA recomputes the global norm from the (L2-resident) gradient in
@@ -442,10 +425,7 @@ __global__ void __launch_bounds__(256) clip_adam_kernel(AdamArgs a) {
     if (threadIdx.x == 0) {
         double t = 0.0;
         for (int w = 0; w < 8; ++w) t += sh[w];
-        const float norm = (float)sqrt(t);
-        const float c = a.max_norm / (norm + 1e-6f);
-        s_coef = c < 1.0f ? c : 1.0f;
-        if (blockIdx.x == 0 && a.norm_out) *a.norm_out = norm;
+        s_coef = clip_coef(t, a);
     }
     __syncthreads();
     const float coef = s_coef;
@@ -453,48 +433,29 @@ __global__ void __launch_bounds__(256) clip_adam_kernel(AdamArgs a) {
     if (i >= a.P) return;
     const float gsc = (a.grad[i] * a.grad_scale) * coef;
     float m = a.m[i], v = a.v[i], p = a.params[i];
-    m = m + a.om_beta1 * (gsc - m);                        // exp_avg.lerp_(grad, 1 - beta1)
-    v = v * a.beta2 + (a.om_beta2 * gsc) * gsc;            // exp_avg_sq.mul_(beta2).addcmul_(grad, grad, 1 - beta2)
-    const float denom = sqrtf(v) / a.bc2_sqrt + a.eps;
-    p = p + (a.neg_step_size * m) / denom;                 // param.addcdiv_(exp_avg, denom, value=-step_size)
+    adam_apply(gsc, m, v, p, a.om_beta1, a.beta2, a.om_beta2, a.eps, a.neg_step_size, a.bc2_sqrt);
     a.m[i] = m; a.v[i] = v; a.params[i] = p;
     if (a.packed != nullptr) packed_store_any<O, A, HID>(a.packed, i, p);
 }
 
-// Single-GPU tail of a minibatch step in ONE cooperative launch: fixed-order fold of the per-CTA partial gradients,
-// global-norm clip and Adam (+ packed-layout refresh).  blockDim = (32, 8): a CTA owns 32 parameters, thread (x, y)
-// folds partials y, y+8, ...; after a grid-wide barrier (all CTAs are co-resident: cooperative launch) every CTA
-// sums the per-CTA squared norms in the same order and applies Adam to its 32 parameters.
-struct FusedArgs {
-    AdamArgs a;
-    const float* grad_part; const float* loss_part; float* grad_out; float* loss_terms_out;
-    double* cta_sumsq; uint32_t* arrive; uint32_t* depart;
-    int nparts, ppad;
-    uint32_t mb_count;
-    float ent_coef, vf_coef;
-};
-
+// Single-GPU tail of a minibatch step in ONE cooperative launch: fixed-order fold of the `nparts` per-CTA partial
+// gradients, global-norm clip and Adam (+ packed-layout refresh), with the arguments of the tensor-core fused step (g.tail).
+// blockDim = (32, 8): a CTA owns 32 parameters, thread (x, y) folds slice y of the partials; after a grid-wide barrier on
+// tail.ctr[0] (all CTAs are co-resident: cooperative launch) every CTA sums the per-CTA squared norms in the same order and
+// applies Adam to its 32 parameters.
 template <int O, int A>
-__global__ void __launch_bounds__(256) reduce_clip_adam_kernel(FusedArgs f) {
+__global__ void __launch_bounds__(256) reduce_clip_adam_kernel(const __grid_constant__ GradArgs g, int nparts) {
     __shared__ float sh[8][33];
     __shared__ double shd[32];
     __shared__ float s_coef;
-    const int P = f.a.P;
+    const TailArgs& tl = g.tail;
+    const AdamArgs& a = tl.a;
+    uint32_t* const arrive = tl.ctr;
+    uint32_t* const depart = tl.ctr + 3;
+    const int P = a.P;
     const int p = blockIdx.x * 32 + threadIdx.x;
     float sacc = 0.0f;
-    if (p < P) {
-        float a0 = 0.f, a1 = 0.f, a2 = 0.f, a3 = 0.f;
-        int c = threadIdx.y;
-        for (; c + 24 < f.nparts; c += 32) {
-            const float v0 = __ldcg(f.grad_part + (size_t)c * f.ppad + p);
-            const float v1 = __ldcg(f.grad_part + (size_t)(c + 8) * f.ppad + p);
-            const float v2 = __ldcg(f.grad_part + (size_t)(c + 16) * f.ppad + p);
-            const float v3 = __ldcg(f.grad_part + (size_t)(c + 24) * f.ppad + p);
-            a0 += v0; a1 += v1; a2 += v2; a3 += v3;
-        }
-        for (; c < f.nparts; c += 8) a0 += __ldcg(f.grad_part + (size_t)c * f.ppad + p);
-        sacc = (a0 + a1) + (a2 + a3);
-    }
+    if (p < P) sacc = fold_partials(g.grad_part, g.ppad, p, threadIdx.y, 1, nparts);
     sh[threadIdx.y][threadIdx.x] = sacc;
     __syncthreads();
     float gval = 0.0f;
@@ -503,63 +464,42 @@ __global__ void __launch_bounds__(256) reduce_clip_adam_kernel(FusedArgs f) {
 #pragma unroll
         for (int y = 1; y < 8; ++y) t += sh[y][threadIdx.x];
         gval = p < P ? t : 0.0f;
-        if (p < P) f.grad_out[p] = gval;
-        const double gs = (double)(gval * f.a.grad_scale);
+        if (p < P) tl.grad_out[p] = gval;
+        const double gs = (double)(gval * a.grad_scale);
         shd[threadIdx.x] = gs * gs;
     }
-    if (blockIdx.x == 0 && threadIdx.y == 1 && threadIdx.x < 5 && f.loss_terms_out != nullptr) {
-        float t = 0.f;
-        for (int c = 0; c < f.nparts; ++c) t += __ldcg(f.loss_part + c * LOSS_TERMS + threadIdx.x);
-        const float inv = 1.0f / (float)f.mb_count;
-        const float t0 = __shfl_sync(0x1fu, t, 0), t1 = __shfl_sync(0x1fu, t, 1), t2 = __shfl_sync(0x1fu, t, 2);
-        const float t3 = __shfl_sync(0x1fu, t, 3), t4 = __shfl_sync(0x1fu, t, 4);
-        if (threadIdx.x == 0) {
-            const float pg = t0 * inv, vl = 0.5f * t1 * inv, en = t2 * inv;
-            f.loss_terms_out[0] = pg - f.ent_coef * en + vl * f.vf_coef;
-            f.loss_terms_out[1] = pg; f.loss_terms_out[2] = vl; f.loss_terms_out[3] = en;
-            f.loss_terms_out[4] = t3 * inv; f.loss_terms_out[5] = t4 * inv;
-            f.loss_terms_out[6] = 0.0f; f.loss_terms_out[7] = 0.0f;
-        }
-    }
+    if (blockIdx.x == 0 && threadIdx.y == 1 && threadIdx.x < 5 && tl.loss_terms_out != nullptr)
+        fold_loss_terms(g.loss_part, nparts, g.mb_count, g.ent_coef, g.vf_coef, tl.loss_terms_out);
     __syncthreads();
     // ---- grid-wide barrier, then every CTA folds the per-CTA squared norms in the same (lane-strided) order ----
     if (threadIdx.y == 0) {
         double t = shd[threadIdx.x];
         t = warp_sum(t);
         if (threadIdx.x == 0) {
-            f.cta_sumsq[blockIdx.x] = t;
+            tl.cta_sumsq[blockIdx.x] = t;
             __threadfence();
-            atomicAdd(f.arrive, 1u);
-            while (*reinterpret_cast<volatile uint32_t*>(f.arrive) < gridDim.x) { }
+            atomicAdd(arrive, 1u);
+            while (*reinterpret_cast<volatile uint32_t*>(arrive) < gridDim.x) { }
             __threadfence();
         }
         __syncwarp();
         double tot = 0.0;
-        for (unsigned i = threadIdx.x; i < gridDim.x; i += 32) tot += __ldcg(f.cta_sumsq + i);
+        for (unsigned i = threadIdx.x; i < gridDim.x; i += 32) tot += __ldcg(tl.cta_sumsq + i);
         tot = warp_sum(tot);
-        if (threadIdx.x == 0) {
-            const float norm = (float)sqrt(tot);
-            const float cf = f.a.max_norm / (norm + 1e-6f);
-            s_coef = cf < 1.0f ? cf : 1.0f;
-            if (blockIdx.x == 0 && f.a.norm_out) *f.a.norm_out = norm;
-        }
+        if (threadIdx.x == 0) s_coef = clip_coef(tot, a);
     }
     __syncthreads();
     if (threadIdx.y == 0 && p < P) {
-        const AdamArgs& a = f.a;
         const float gsc = (gval * a.grad_scale) * s_coef;
         float m = a.m[p], v = a.v[p], w = a.params[p];
-        m = m + a.om_beta1 * (gsc - m);
-        v = v * a.beta2 + (a.om_beta2 * gsc) * gsc;
-        const float denom = sqrtf(v) / a.bc2_sqrt + a.eps;
-        w = w + (a.neg_step_size * m) / denom;
+        adam_apply(gsc, m, v, w, a.om_beta1, a.beta2, a.om_beta2, a.eps, a.neg_step_size, a.bc2_sqrt);
         a.m[p] = m; a.v[p] = v; a.params[p] = w;
         if (a.packed != nullptr) packed_store<O, A>(a.packed, p, w);
     }
     __syncthreads();
     if (threadIdx.x == 0 && threadIdx.y == 0) {
         __threadfence();
-        if (atomicAdd(f.depart, 1u) == gridDim.x - 1) { *f.arrive = 0u; *f.depart = 0u; }   // re-arm (stream-ordered)
+        if (atomicAdd(depart, 1u) == gridDim.x - 1) { *arrive = 0u; *depart = 0u; }   // re-arm (stream-ordered)
     }
 }
 
@@ -574,12 +514,22 @@ int launch_grad(const GradArgs& g, int P, float* grad_out, float* loss_terms_out
     ppo_grad_kernel<O, A, OP, RW><<<grid, GT, smem, st>>>(g);
     DRL_LAUNCH_CHECK("ppo_grad_kernel");
     if (grid_out != nullptr) { *grid_out = grid; return DRL_OK; }   // caller folds the partials itself
-    return launch_grad_reduce(g, grid, P, grad_out, loss_terms_out, st);
+    return launch_grad_reduce(g, grid, P, 1, P, grad_out, loss_terms_out, st);
 }
 
-int launch_grad_reduce(const GradArgs& g, int grid, int P, float* grad_out, float* loss_terms_out, cudaStream_t st) {
-    grad_reduce_kernel<<<(P + 31) / 32, dim3(32, 8), 0, st>>>(g.grad_part, g.loss_part, grid, g.ppad, P, g.mb_count, g.ent_coef,
-                                                       g.vf_coef, grad_out, loss_terms_out);
+template <int HID>
+static void launch_clip_adam(const drl_net_t* net, const AdamArgs& a, cudaStream_t st) {
+    const int blocks = (a.P + 255) / 256;
+    if (net->obs_dim == 4) clip_adam_kernel<4, 2, HID><<<blocks, 256, 0, st>>>(a);
+    else if (net->obs_dim == 2) clip_adam_kernel<2, 3, HID><<<blocks, 256, 0, st>>>(a);
+    else clip_adam_kernel<6, 3, HID><<<blocks, 256, 0, st>>>(a);
+}
+
+int launch_grad_reduce(const GradArgs& g, int nrows, int P, int stride, int critic0, float* grad_out, float* loss_terms_out,
+                       cudaStream_t st) {
+    const auto kernel = stride == 2 ? grad_reduce_kernel<2> : grad_reduce_kernel<1>;
+    kernel<<<(P + 31) / 32, dim3(32, 8), 0, st>>>(g.grad_part, g.loss_part, nrows, g.ppad, P, critic0, g.mb_count, g.ent_coef,
+                                                  g.vf_coef, grad_out, loss_terms_out);
     DRL_LAUNCH_CHECK("grad_reduce_kernel");
     return DRL_OK;
 }
@@ -626,11 +576,9 @@ static void fill_adam(AdamArgs& a, const drl_net_t* net, float* params, const fl
     a.P = (int)drl_param_count(net);
     a.grad_scale = (float)grad_scale; a.max_norm = (float)max_grad_norm;
     a.beta2 = (float)beta2; a.om_beta1 = (float)(1.0 - beta1); a.om_beta2 = (float)(1.0 - beta2); a.eps = (float)eps;
-    // scalars exactly as torch.optim.adam._single_tensor_adam computes them (Python floats, fp64)
-    const double bc1 = 1.0 - pow(beta1, (double)step);
-    const double bc2 = 1.0 - pow(beta2, (double)step);
-    a.neg_step_size = (float)(-(lr / bc1));
-    a.bc2_sqrt = (float)sqrt(bc2);
+    const AdamScalars s = adam_scalars(step, lr, beta1, beta2);
+    a.neg_step_size = s.neg_step_size;
+    a.bc2_sqrt = s.bc2_sqrt;
 }
 
 int drl_ppo_minibatch_grad(const drl_net_t* net, const float* packed, const float* rec, const uint32_t* idx,
@@ -658,50 +606,39 @@ static int minibatch_update_impl(const drl_net_t* net, float* packed, const floa
     DRL_REQUIRE(num_steps == 1 || (flags & DRL_GRAD_TENSOR_CORES), "drl_ppo_minibatch_update: num_steps > 1 needs the tensor-core path");
     DRL_REQUIRE(ctrl == nullptr || ordinal + num_steps <= DRL_CTRL_MAX_STEPS, "drl_ppo_minibatch_update: ordinal %d + %d steps > %d", ordinal,
                 num_steps, DRL_CTRL_MAX_STEPS);
+    const bool tc = flags & DRL_GRAD_TENSOR_CORES;
+    DRL_REQUIRE(tc || comm == nullptr, "drl_ppo_minibatch_update: the fp32 path has no fused multi-GPU form");
     cudaStream_t st = as_stream(stream);
     GradArgs g;
     int grid = 0;
-    const WorkspaceLayout w = workspace_layout(drl_param_count(net));
-    if (flags & DRL_GRAD_TENSOR_CORES) {   // one cooperative launch: gradient + fold + [peer all-reduce] + clip + Adam
-        rc = run_grad(net, packed, rec, idx, mb_start, mb_count, adv_stats, coef, grad_out, loss_terms_out, workspace, workspace_bytes,
-                      flags, st, &g, nullptr);
-        if (rc != DRL_OK) return rc;
-        const int world = comm ? comm->world : 1;
-        g.tail.enabled = 1;
-        fill_adam(g.tail.a, net, params, grad_out, exp_avg, exp_avg_sq, step, lr, beta1, beta2, eps, max_grad_norm, 1.0 / world, packed,
-                  norm_out);
-        g.tail.grad_out = grad_out; g.tail.loss_terms_out = loss_terms_out;
-        g.tail.cta_sumsq = reinterpret_cast<double*>((char*)workspace + w.cta_sumsq);
-        g.tail.ctr = reinterpret_cast<uint32_t*>((char*)workspace + w.counters) + 8;
-        g.tail.world = world; g.tail.rank = comm ? comm->rank : 0; g.tail.seq = comm ? comm->seq : 0;
-        g.tail.error_flag = comm ? comm->error_flag : nullptr;
-        g.tail.ctrl = ctrl; g.tail.ordinal = ordinal;
-        g.tail.nsteps = num_steps;
-        for (int sidx = 0; sidx < num_steps; ++sidx) {      // by-value Adam scalars of optimizer steps step .. step + num_steps - 1
-            AdamArgs tmp;
-            fill_adam(tmp, net, params, grad_out, exp_avg, exp_avg_sq, step + sidx, lr, beta1, beta2, eps, max_grad_norm, 1.0 / world, packed,
-                      norm_out);
-            g.tail.neg_step_size_s[sidx] = tmp.neg_step_size;
-            g.tail.bc2_sqrt_s[sidx] = tmp.bc2_sqrt;
-        }
-        for (int r = 0; r < DRL_MAX_RANKS; ++r)
-            g.tail.peer[r] = (comm && r < world) ? reinterpret_cast<unsigned char*>(comm->peer[r]) : nullptr;
-        return launch_grad_tc_fused(net, g, st);
-    }
-    DRL_REQUIRE(comm == nullptr, "drl_ppo_minibatch_update: the fp32 path has no fused multi-GPU form");
+    // tcgen05: arguments only, the gradient and its tail are one cooperative launch (gradient + fold + [peer all-reduce] + clip
+    // + Adam).  fp32: launches the gradient kernel; reduce_clip_adam_kernel (fold + clip + Adam) then reads the same g.tail.
     rc = run_grad(net, packed, rec, idx, mb_start, mb_count, adv_stats, coef, grad_out, loss_terms_out, workspace, workspace_bytes,
-                  flags, st, &g, &grid);
+                  flags, st, &g, tc ? nullptr : &grid);
     if (rc != DRL_OK) return rc;
-    FusedArgs f;
-    fill_adam(f.a, net, params, grad_out, exp_avg, exp_avg_sq, step, lr, beta1, beta2, eps, max_grad_norm, 1.0, packed, norm_out);
-    f.grad_part = g.grad_part; f.loss_part = g.loss_part; f.grad_out = grad_out; f.loss_terms_out = loss_terms_out;
-    f.cta_sumsq = reinterpret_cast<double*>((char*)workspace + w.cta_sumsq);
-    f.arrive = reinterpret_cast<uint32_t*>((char*)workspace + w.counters) + 4;
-    f.depart = f.arrive + 1;
-    f.nparts = grid; f.ppad = g.ppad; f.mb_count = mb_count; f.ent_coef = coef->ent_coef; f.vf_coef = coef->vf_coef;
-    const int blocks = (f.a.P + 31) / 32;
-    DRL_REQUIRE(blocks <= 1024, "drl_ppo_minibatch_update: %d parameters exceed the squared-norm scratch", f.a.P);
-    void* args[] = {&f};
+    const WorkspaceLayout w = workspace_layout(drl_param_count(net));
+    const int world = comm ? comm->world : 1;
+    g.tail.enabled = 1;
+    fill_adam(g.tail.a, net, params, grad_out, exp_avg, exp_avg_sq, step, lr, beta1, beta2, eps, max_grad_norm, 1.0 / world, packed,
+              norm_out);
+    g.tail.grad_out = grad_out; g.tail.loss_terms_out = loss_terms_out;
+    g.tail.cta_sumsq = reinterpret_cast<double*>((char*)workspace + w.cta_sumsq);
+    g.tail.ctr = reinterpret_cast<uint32_t*>((char*)workspace + w.counters) + 8;
+    g.tail.world = world; g.tail.rank = comm ? comm->rank : 0; g.tail.seq = comm ? comm->seq : 0;
+    g.tail.error_flag = comm ? comm->error_flag : nullptr;
+    g.tail.ctrl = ctrl; g.tail.ordinal = ordinal;
+    g.tail.nsteps = num_steps;
+    for (int sidx = 0; sidx < num_steps; ++sidx) {      // by-value Adam scalars of optimizer steps step .. step + num_steps - 1
+        const AdamScalars s = adam_scalars(step + sidx, lr, beta1, beta2);
+        g.tail.neg_step_size_s[sidx] = s.neg_step_size;
+        g.tail.bc2_sqrt_s[sidx] = s.bc2_sqrt;
+    }
+    for (int r = 0; r < DRL_MAX_RANKS; ++r)
+        g.tail.peer[r] = (comm && r < world) ? reinterpret_cast<unsigned char*>(comm->peer[r]) : nullptr;
+    if (tc) return launch_grad_tc_fused(net, g, st);
+    const int blocks = (g.tail.a.P + 31) / 32;
+    DRL_REQUIRE(blocks <= 1024, "drl_ppo_minibatch_update: %d parameters exceed the squared-norm scratch", g.tail.a.P);
+    void* args[] = {&g, &grid};
     const void* fn = net->obs_dim == 4 ? (const void*)reduce_clip_adam_kernel<4, 2>
                      : net->obs_dim == 2 ? (const void*)reduce_clip_adam_kernel<2, 3> : (const void*)reduce_clip_adam_kernel<6, 3>;
     DRL_CUDA(cudaLaunchCooperativeKernel(fn, dim3(blocks), dim3(32, 8), args, 0, st));
@@ -767,10 +704,10 @@ int drl_ctrl_set(drl_ctrl_t* ctrl, uint64_t env_step, uint32_t epoch_ctr, uint32
     drl_ctrl_t v;
     memset(&v, 0, sizeof(v));
     v.env_step = env_step; v.epoch_ctr = epoch_ctr; v.comm_seq = comm_seq; v.adam_step = adam_step;
-    for (int k = 0; k < n_steps; ++k) {      // the scalars of fill_adam, for optimizer steps adam_step + 1 ... adam_step + n_steps
-        const double step = (double)(adam_step + k + 1);
-        v.neg_step_size[k] = (float)(-(lr / (1.0 - pow(beta1, step))));
-        v.bc2_sqrt[k] = (float)sqrt(1.0 - pow(beta2, step));
+    for (int k = 0; k < n_steps; ++k) {      // optimizer steps adam_step + 1 ... adam_step + n_steps
+        const AdamScalars s = adam_scalars(adam_step + k + 1, lr, beta1, beta2);
+        v.neg_step_size[k] = s.neg_step_size;
+        v.bc2_sqrt[k] = s.bc2_sqrt;
     }
     ctrl_set_kernel<<<1, DRL_CTRL_MAX_STEPS, 0, as_stream(stream)>>>(ctrl, v);
     DRL_LAUNCH_CHECK("ctrl_set_kernel");
@@ -819,17 +756,8 @@ int drl_clip_adam(const drl_net_t* net, float* params, const float* grad, float*
     DRL_REQUIRE(step >= 1, "drl_clip_adam: step=%lld must be >= 1", (long long)step);
     AdamArgs a;
     fill_adam(a, net, params, grad, exp_avg, exp_avg_sq, step, lr, beta1, beta2, eps, max_grad_norm, grad_scale, packed_out, norm_out);
-    const int blocks = (a.P + 255) / 256;
-    if (net->hidden == 256) {
-        if (net->obs_dim == 4) clip_adam_kernel<4, 2, 256><<<blocks, 256, 0, as_stream(stream)>>>(a);
-        else if (net->obs_dim == 2) clip_adam_kernel<2, 3, 256><<<blocks, 256, 0, as_stream(stream)>>>(a);
-        else clip_adam_kernel<6, 3, 256><<<blocks, 256, 0, as_stream(stream)>>>(a);
-        DRL_LAUNCH_CHECK("clip_adam_kernel");
-        return DRL_OK;
-    }
-    if (net->obs_dim == 4) clip_adam_kernel<4, 2><<<blocks, 256, 0, as_stream(stream)>>>(a);
-    else if (net->obs_dim == 2) clip_adam_kernel<2, 3><<<blocks, 256, 0, as_stream(stream)>>>(a);
-    else clip_adam_kernel<6, 3><<<blocks, 256, 0, as_stream(stream)>>>(a);
+    if (net->hidden == 256) launch_clip_adam<256>(net, a, as_stream(stream));
+    else launch_clip_adam<64>(net, a, as_stream(stream));
     DRL_LAUNCH_CHECK("clip_adam_kernel");
     return DRL_OK;
 }

@@ -237,12 +237,7 @@ __device__ __noinline__ void tc_tail_step(const TailCtx* cx, uint32_t s, uint32_
         double tot = 0.0;
         for (int i = lane; i < nparts; i += 32) tot += __ldcg(tl.cta_sumsq + i);
         tot = warp_sum(tot);
-        if (lane == 0) {
-            const float norm = (float)sqrt(tot);
-            const float cf = ad.max_norm / (norm + 1e-6f);
-            sbc[0] = cf < 1.0f ? cf : 1.0f;
-            if (blockIdx.x == 0 && ad.norm_out) *ad.norm_out = norm;
-        }
+        if (lane == 0) sbc[0] = clip_coef(tot, ad);
     } else if (blockIdx.x == 0 && warp >= 1 && warp <= 5 && loss_terms_out != nullptr) {
         float t = 0.f;                                    // warp w folds loss term w-1 over the CTAs
         for (int c = lane; c < nparts; c += 32) t += __ldcg(cx->loss_part + c * LOSS_TERMS + (warp - 1));
@@ -259,22 +254,13 @@ __device__ __noinline__ void tc_tail_step(const TailCtx* cx, uint32_t s, uint32_
         float m, v, wgt;
         if (p == p_first) { m = pre_m; v = pre_v; wgt = pre_w; }
         else { m = ad.m[p]; v = ad.v[p]; wgt = ad.params[p]; }
-        m = m + ad.om_beta1 * (gsc - m);
-        v = v * ad.beta2 + (ad.om_beta2 * gsc) * gsc;
-        const float denom = sqrtf(v) / bc2_sqrt + ad.eps;
-        wgt = wgt + (neg_step_size * m) / denom;
+        adam_apply(gsc, m, v, wgt, ad.om_beta1, ad.beta2, ad.om_beta2, ad.eps, neg_step_size, bc2_sqrt);
         ad.m[p] = m; ad.v[p] = v; ad.params[p] = wgt;
         if (ad.packed != nullptr) packed_store<O, A>(ad.packed, p, wgt);
     }
     TC_KSTAMP(10);
-    if (blockIdx.x == 0 && tid == 0 && loss_terms_out != nullptr) {
-        const float inv = 1.0f / (float)cx->mb_count;
-        const float pg = sbc[4] * inv, vl = 0.5f * sbc[5] * inv, en = sbc[6] * inv;
-        loss_terms_out[0] = pg - cx->ent_coef * en + vl * cx->vf_coef;
-        loss_terms_out[1] = pg; loss_terms_out[2] = vl; loss_terms_out[3] = en;
-        loss_terms_out[4] = sbc[7] * inv; loss_terms_out[5] = sbc[8] * inv;
-        loss_terms_out[6] = 0.0f; loss_terms_out[7] = 0.0f;
-    }
+    if (blockIdx.x == 0 && tid == 0 && loss_terms_out != nullptr)
+        store_loss_terms(loss_terms_out, sbc + 4, cx->mb_count, cx->ent_coef, cx->vf_coef);
     if (s + 1 < nsteps) {
         // next minibatch of the launch: every CTA has applied its slice of the Adam step (and refreshed its part of the packed
         // weights) -> reload the weight tiles; the loader has the first [obs|1] tiles in the ring already
@@ -877,7 +863,7 @@ static int launch_tc(const GradArgs& g, int P, float* grad_out, float* loss_term
     ppo_grad_tc_kernel<O, A, OP, RW><<<grid, GRAD_TC_BLOCK, smem, st>>>(g);
     DRL_LAUNCH_CHECK("ppo_grad_tc_kernel");
     if (grid_out != nullptr) { *grid_out = grid; return DRL_OK; }
-    return launch_grad_reduce(g, grid, P, grad_out, loss_terms_out, st);
+    return launch_grad_reduce(g, grid, P, 1, P, grad_out, loss_terms_out, st);
 }
 
 int launch_grad_tc(const drl_net_t* net, const GradArgs& g, int P, float* grad_out, float* loss_terms_out, cudaStream_t st,

@@ -37,6 +37,8 @@ from .envs import VecEnv
 from .evaluate import EvalResult, evaluate as _evaluate
 
 EVAL_SEED_OFFSET = 0x9E3779B97F4A7C15     # default evaluation key = (cfg.seed + this) mod 2^64: never a training key
+ADAM_BETAS = (0.9, 0.999)                 # optim.Adam(lr, eps=1e-5) of the reference (ppo.py:90), torch's default betas
+ADAM_EPS = 1e-5
 
 
 def eval_seed(seed: int) -> int:
@@ -369,7 +371,7 @@ class PPOTrainer:
                             net, self.agent.packed.data_ptr(), self.records.data_ptr(), idx_ptr, start, count,
                             stats_ptr + 8 * k, C.byref(self.coef), self.agent.flat_params.data_ptr(),
                             self.grad.data_ptr(), self.exp_avg.data_ptr(), self.exp_avg_sq.data_ptr(), self.ctrl.data_ptr(), row,
-                            0.9, 0.999, 1e-5, cfg.max_grad_norm, self.loss_terms.data_ptr() + 32 * row,
+                            *ADAM_BETAS, ADAM_EPS, cfg.max_grad_norm, self.loss_terms.data_ptr() + 32 * row,
                             self.grad_norm.data_ptr(), self.workspace.data_ptr(), self.ws_bytes, self.grad_flags,
                             C.byref(self.peer.struct) if self.peer is not None else None, ns, st))
                     self.kernel_launches += 1
@@ -386,7 +388,7 @@ class PPOTrainer:
                             net, self.agent.packed.data_ptr(), self.records.data_ptr(), idx_ptr, start, count,
                             stats_ptr + 8 * k, C.byref(self.coef), self.agent.flat_params.data_ptr(),
                             self.grad.data_ptr(), self.exp_avg.data_ptr(), self.exp_avg_sq.data_ptr(), first_step, lr,
-                            0.9, 0.999, 1e-5, cfg.max_grad_norm, self.loss_terms.data_ptr() + 32 * row,
+                            *ADAM_BETAS, ADAM_EPS, cfg.max_grad_norm, self.loss_terms.data_ptr() + 32 * row,
                             self.grad_norm.data_ptr(), self.workspace.data_ptr(), self.ws_bytes, self.grad_flags,
                             C.byref(comm), ns, st))
                     comm.seq = self.peer.seq
@@ -400,7 +402,7 @@ class PPOTrainer:
                             net, self.agent.packed.data_ptr(), self.records.data_ptr(), idx_ptr, start, count,
                             stats_ptr + 8 * k, C.byref(self.coef), self.agent.flat_params.data_ptr(),
                             self.grad.data_ptr(), self.exp_avg.data_ptr(), self.exp_avg_sq.data_ptr(), first_step, lr,
-                            0.9, 0.999, 1e-5, cfg.max_grad_norm, self.loss_terms.data_ptr() + 32 * row,
+                            *ADAM_BETAS, ADAM_EPS, cfg.max_grad_norm, self.loss_terms.data_ptr() + 32 * row,
                             self.grad_norm.data_ptr(), self.workspace.data_ptr(), self.ws_bytes, self.grad_flags, ns, st))
                     self.kernel_launches += 1 if self.grad_flags == 1 else 2
                     continue
@@ -416,7 +418,7 @@ class PPOTrainer:
                 with _Phase(self, "clip_adam"):
                     _lib.check(self.L.drl_clip_adam(net, self.agent.flat_params.data_ptr(), self.grad.data_ptr(),
                                                     self.exp_avg.data_ptr(), self.exp_avg_sq.data_ptr(), self.adam_step, lr,
-                                                    0.9, 0.999, 1e-5, cfg.max_grad_norm, 1.0 / self.world,
+                                                    *ADAM_BETAS, ADAM_EPS, cfg.max_grad_norm, 1.0 / self.world,
                                                     self.agent.packed.data_ptr(), self.grad_norm.data_ptr(), st))
                 self.kernel_launches += 3
 
@@ -439,7 +441,7 @@ class PPOTrainer:
             cfg = self.cfg
             n_opt = cfg.update_epochs * self.n_mb
             _lib.check(self.L.drl_ctrl_set(self.ctrl.data_ptr(), self.env.step_count, self.update_idx * cfg.update_epochs,
-                                           self.peer.seq if self.peer is not None else 0, self.adam_step, n_opt, lr, 0.9, 0.999,
+                                           self.peer.seq if self.peer is not None else 0, self.adam_step, n_opt, lr, *ADAM_BETAS,
                                            _lib.stream_ptr()))
             if self._graph is None and self._graph_warm >= 2:
                 self._capture_graph(lr)
